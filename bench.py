@@ -24,6 +24,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True    # runs from the built tree, which may be read-only: nothing is written into it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -92,7 +93,6 @@ def cpu_reference_rate(blob, chunk, level, threads, seconds=0.0):
     its contiguous share once (seconds = 0: a single un-looped pass) or repeatedly until `seconds` have passed.
     Returns (GB/s, wall seconds, ratio)."""
     import helpers as H
-    H.build_oracle()
     L = H.oracle()
     from concurrent.futures import ThreadPoolExecutor
     c = ctypes
@@ -133,6 +133,26 @@ def make_data(nbytes, device, seed):
     return H.synth_text_torch(nbytes, device, seed=seed)
 
 
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 7
+
+
+def dump_outputs(path, dst, sizes, suffix=""):
+    """Writes what the timed encode returned in its last step, so that two builds can be compared output for output:
+    sizes.npy (every frame's size, float64), frames.npy (the frame bytes of a fixed, seeded sample of chunks, one row of
+    `slot` float32 values per chunk, zero past the frame's end) and frame_index.npy (the sampled chunks), 64 MB at most."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    n, slot = dst.shape
+    k = max(0, min(n, 64, (DUMP_BYTES - 16 * n) // (4 * slot)))
+    idx = np.sort(np.random.Generator(np.random.PCG64(DUMP_SEED)).choice(n, size=k, replace=False))
+    rows = dst[torch.from_numpy(idx).to(dst.device)].cpu().numpy()
+    rows[np.arange(slot)[None, :] >= sizes[idx][:, None]] = 0
+    np.save(os.path.join(path, "sizes%s.npy" % suffix), sizes.astype(np.float64))
+    np.save(os.path.join(path, "frame_index%s.npy" % suffix), idx.astype(np.float64))
+    np.save(os.path.join(path, "frames%s.npy" % suffix), rows.astype(np.float32))
+
+
 def pci_bus_id(index):
     try:
         out = subprocess.run(["nvidia-smi", "-i", str(index), "--query-gpu=pci.bus_id", "--format=csv,noheader"],
@@ -153,7 +173,13 @@ def main():
     ap.add_argument("--e2e-chunks", type=int, default=0, help="chunks per e2e step (default: all)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the decode / S2 / huff0 / chunk-API side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's frames and all "
+                                                          "frame sizes to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU encoder's outputs; --impl reference keeps none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -240,6 +266,8 @@ def main():
     enc.profile(False)
     outs_h = outs.cpu().numpy()
     assert (outs_h > 0).all(), "encode error"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dst, outs_h, "" if world == 1 else "_rank%d" % rank)
     out_bytes = int(outs_h.sum())
     in_bytes = n * CHUNK
     peak, peak_kind = hbm_peak()

@@ -11,8 +11,6 @@ import pytest
 
 import helpers as H
 
-REF = "/root/reference/zstd/testdata"
-
 
 def _pairs(zf):
     names = set(zf.namelist())
