@@ -25,8 +25,9 @@
 // from a per-CTA scratch array -> extend forwards/backwards -> emit -> skip), neighbours are merged by a prefix
 // maximum of match ends (as in round 1), sequences and codes are written, and the literals are produced by a
 // warp-cooperative stream compaction of the staged chunk under a one-bit-per-position literal mask (coalesced byte
-// stores; no 64 KiB literal staging buffer, which is what lets two CTAs share an SM).  The literal and code histograms
-// moved to their own kernel (b2c_zstd_hist_kernel).
+// stores; no 64 KiB literal staging buffer, which is what lets two CTAs share an SM).  The literal and sequence-code
+// histograms are counted on the way, with shared-memory atomics into 1.8 KB of the per-thread arrays that are dead by
+// then (see LZ_HIST_WORDS), so no later pass has to read the literals and codes back.
 #pragma once
 #include "b2c_zstd_enc.cuh"
 
@@ -136,6 +137,11 @@ template <int LV> struct LzLayout {
 static_assert(2 * (LzLayout<1>::SMEM_BYTES + 1024) <= 228 * 1024, "two level-1 parse CTAs must fit one SM");
 static_assert(LzLayout<2>::SMEM_BYTES <= 227 * 1024 && LzLayout<5>::SMEM_BYTES <= 227 * 1024, "the level-2 / level-3 parse CTA must fit one SM");
 static_assert(2 * (LzLayout<3>::SMEM_BYTES + 1024) <= 228 * 1024 && 2 * (LzLayout<4>::SMEM_BYTES + 1024) <= 228 * 1024, "two S2 parse CTAs must fit one SM");
+// zstd histograms of a chunk: 256 literal counters + 3 x 64 sequence-code counters, u32, in the longLen array
+// of SM_ARR (NT words; last read before the merge scan, see lz_parse_chunk)
+constexpr uint32_t LZ_HIST_WORDS = 256 + 3 * 64;
+static_assert(LzCfg<1>::NT >= (int)LZ_HIST_WORDS && LzCfg<2>::NT >= (int)LZ_HIST_WORDS && LzCfg<5>::NT >= (int)LZ_HIST_WORDS,
+              "the zstd histograms must fit the longLen array");
 
 // hashes: two 32-bit multiply-adds (the reference's hashLen is a 64-bit multiply, zstd/hash.go:27-33; table contents
 // are an implementation detail, only verified matches reach the output)
@@ -553,6 +559,10 @@ B2C_DEV void lz_parse_chunk(uint8_t *smem, const ZstdEncParams &P, uint32_t chun
     // ---------------------------------------------------------------- P4: merge (trim overlaps), global layout
     uint32_t dummyTotal;
     const uint32_t R = group_scan_excl_max(lastE, sh->ws, 0, NT, tid, &dummyTotal);   // everything before R is taken
+    // the zstd histograms live in longLen, whose last read (myLong) precedes the barriers of the scan above;
+    // the barrier before the next scan orders this zeroing before the counting in P5 / P6
+    uint32_t *const hcnt = longLen;             // [0, 256) literal bytes | 256 + 64 * table + code
+    if constexpr (ZSTD) { if (tid < LZ_HIST_WORDS) hcnt[tid] = 0; }
     B2C_PHASE(8);
     // A record survives when at least 4 of its bytes lie behind R; the dropped ones are a prefix of the thread's records
     // (records are ordered and disjoint), so the kept ones are firstKept .. cnt-1, the first of them possibly trimmed.
@@ -783,9 +793,15 @@ B2C_DEV void lz_parse_chunk(uint8_t *smem, const ZstdEncParams &P, uint32_t chun
                     const bool isrep = (gi > 0) && (d0 == pd) && (ll > 0);
                     const uint32_t ofv = isrep ? 1u : d0 + 3;
                     wlen.put(gi, ll, l2 - 3); wof[gi] = ofv;
-                    wcodes[TBL_LL * mseq + gi] = (uint8_t)seq_ll_code(ll);
-                    wcodes[TBL_OF * mseq + gi] = (uint8_t)highbit32(ofv);
-                    wcodes[TBL_ML * mseq + gi] = (uint8_t)seq_ml_code(l2 - 3);
+                    const uint32_t cll = seq_ll_code(ll), cof = highbit32(ofv), cml = seq_ml_code(l2 - 3);
+                    wcodes[TBL_LL * mseq + gi] = (uint8_t)cll;
+                    wcodes[TBL_OF * mseq + gi] = (uint8_t)cof;
+                    wcodes[TBL_ML * mseq + gi] = (uint8_t)cml;
+                    if (kind == 0) {      // (only compressed candidates use the histograms)
+                        atomicAdd(&hcnt[256 + 64 * TBL_LL + cll], 1u);
+                        atomicAdd(&hcnt[256 + 64 * TBL_OF + cof], 1u);
+                        atomicAdd(&hcnt[256 + 64 * TBL_ML + cml], 1u);
+                    }
                 }
                 carryE = __shfl_sync(FULLMASK, e0, 31); carryD = __shfl_sync(FULLMASK, d0, 31);
             }
@@ -850,9 +866,10 @@ B2C_DEV void lz_parse_chunk(uint8_t *smem, const ZstdEncParams &P, uint32_t chun
                     const uint32_t packed = __byte_perm(v, 0u, (uint32_t)plut[nib[q]]);
                     uint8_t *o = stg + rbase + ((incl >> (8 * q)) & 0xffu) - c;
                     o[0] = (uint8_t)packed;
-                    if (c > 1) o[1] = (uint8_t)(packed >> 8);
-                    if (c > 2) o[2] = (uint8_t)(packed >> 16);
-                    if (c > 3) o[3] = (uint8_t)(packed >> 24);
+                    atomicAdd(&hcnt[packed & 0xffu], 1u);
+                    if (c > 1) { o[1] = (uint8_t)(packed >> 8); atomicAdd(&hcnt[(packed >> 8) & 0xffu], 1u); }
+                    if (c > 2) { o[2] = (uint8_t)(packed >> 16); atomicAdd(&hcnt[(packed >> 16) & 0xffu], 1u); }
+                    if (c > 3) { o[3] = (uint8_t)(packed >> 24); atomicAdd(&hcnt[packed >> 24], 1u); }
                 }
                 rbase += (tots >> (8 * q)) & 0xffu;
             }
@@ -862,142 +879,64 @@ B2C_DEV void lz_parse_chunk(uint8_t *smem, const ZstdEncParams &P, uint32_t chun
 #undef REC
     if (tid == 0) { W->n = nblk; W->nseq = nseq; W->nlit = nlit; W->kind = kind; W->rleLen = sh->rleLen; }
     __syncthreads();
+    if (kind == 0) {
+        // histograms of a compressed candidate (zstd_tables_chunk reads them for no other kind); warp t < 3 publishes code
+        // table t and its highest used code
+        for (uint32_t i = tid; i < 256; i += NT) W->litHist[i] = hcnt[i];
+        if (w < 3) {
+            const uint32_t lo = hcnt[256 + 64 * w + lane], hi = hcnt[256 + 64 * w + 32 + lane];
+            W->seqHist[w][lane] = lo; W->seqHist[w][32 + lane] = hi;
+            const unsigned nzLo = __ballot_sync(FULLMASK, lo != 0), nzHi = __ballot_sync(FULLMASK, hi != 0);
+            if (lane == 0)
+                W->maxSym[w] = nzHi ? 32 + (31 - (uint32_t)__clz((int)nzHi)) : (nzLo ? 31 - (uint32_t)__clz((int)nzLo) : 0u);
+        }
+    }
     B2C_PHASE(5);
     }   // zstd mode
 }
 
-// ------------------------------------------------------------------------------------------------ histograms
-// One 128-thread CTA per chunk: literal histogram (one private u8 counter per (symbol, lane) and warp -- no atomics, no
-// races; literals are counted in slices small enough that a counter cannot wrap) and the three sequence-code
-// histograms (ballot counts, lane l owns the codes whose low 5 bits equal l) with their highest used code.  Input:
-// the literals and codes the parse kernel left in the work pool.  (Round 1 did this inside the parse kernel, where it
-// pinned 64 KiB of shared memory; as a separate kernel it runs at seven CTAs per SM.)
+#ifdef B2C_EMU
+// CPU emulator only (tests/emu runs it between the parse and the tables): recounts the histograms of every compressed
+// candidate from the literals and codes in the work pool and compares them, and the highest used codes, with what the
+// parse counted.  A difference turns the chunk into an error (kind 3: its output size is negative), so every test of
+// the emulated encoder fails on it.  The device pipeline has no such pass.
 constexpr int HIST_NT = 128;
-constexpr int HIST_WARPS = HIST_NT / 32;
-constexpr uint32_t HIST_SLICE = 15u * 16u * HIST_NT; // bytes per slice: a lane takes 16-byte pieces, at most 15 of them (240 <= 255)
-constexpr uint32_t HIST_SMEM_BYTES = HIST_WARPS * 256 * 32;
-// Private-counter byte histogram of stream[s0, s1) (s0 a multiple of 16, stream 16-byte aligned): every lane owns one
-// byte counter per symbol (col[sym * 32]), reads 16 bytes per step with the next step's load already in flight, and merges
-// equal symbols inside a word so that the four updates of a word are independent.  At most 255 symbols per lane and call.
-template <uint32_t SYMMASK>
-B2C_DEV void hist_count_stream(const uint8_t *stream, uint32_t s0, uint32_t s1, uint8_t *col, unsigned tid) {
-    const uint4 *s16 = reinterpret_cast<const uint4 *>(stream);
-    const uint32_t n16 = (s1 + 15) / 16;
-    uint32_t i = s0 / 16 + tid;
-    uint4 v = (i < n16) ? B2C_LDG(s16 + i) : make_uint4(0, 0, 0, 0);
-    while (i < n16) {
-        const uint32_t inext = i + HIST_NT;
-        const uint4 vnext = (inext < n16) ? B2C_LDG(s16 + inext) : make_uint4(0, 0, 0, 0);   // requested before this one is used
-        const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-            const uint32_t pos = 16 * i + 4 * k;
-            if (pos < s1) {
-                const uint32_t nv = (pos + 4 <= s1) ? 4u : s1 - pos;
-                const uint32_t x = wv[k];
-                const uint32_t a0 = x & SYMMASK, a1 = (x >> 8) & SYMMASK, a2 = (x >> 16) & SYMMASK, a3 = (x >> 24) & SYMMASK;
-                uint32_t i0 = 1, i1 = nv > 1, i2 = nv > 2, i3 = nv > 3;
-                if (a1 == a0) { i0 += i1; i1 = 0; }
-                if (a2 == a0) { i0 += i2; i2 = 0; } else if (a2 == a1) { i1 += i2; i2 = 0; }
-                if (a3 == a0) { i0 += i3; i3 = 0; } else if (a3 == a1) { i1 += i3; i3 = 0; } else if (a3 == a2) { i2 += i3; i3 = 0; }
-                const uint32_t c0 = col[a0 * 32], c1 = col[a1 * 32], c2 = col[a2 * 32], c3 = col[a3 * 32];
-                col[a0 * 32] = (uint8_t)(c0 + i0);
-                if (i1) col[a1 * 32] = (uint8_t)(c1 + i1);
-                if (i2) col[a2 * 32] = (uint8_t)(c2 + i2);
-                if (i3) col[a3 * 32] = (uint8_t)(c3 + i3);
-            }
-        }
-        i = inext; v = vnext;
-    }
-}
-
+constexpr uint32_t HIST_SMEM_BYTES = LZ_HIST_WORDS * 4 + 16;
 B2C_DEV void zstd_hist_chunk(uint8_t *smem, const ZstdEncParams &P, uint32_t chunk) {
-    const unsigned tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const unsigned tid = threadIdx.x;
     ChunkWork *W = P.work + chunk;
-    const uint32_t nlit = W->nlit, nseq = W->nseq;
-    const uint8_t *lit = wk_lit(P, chunk);
-    if (P.dbg_hdr && W->kind != 3) {
-        const WkLens wlen = wk_lens(P, chunk);
-        const uint32_t *wof = wk_of(P, chunk);
-        for (uint32_t i = tid; i < nseq && i < P.dbg_seq_cap && i < P.maxseq; i += HIST_NT) {
-            uint32_t *d = P.dbg_seqs + ((uint64_t)chunk * P.dbg_seq_cap + i) * 3;
-            d[0] = wlen.get_ll(i); d[1] = wlen.get_ml(i); d[2] = wof[i];
+    uint32_t *h = reinterpret_cast<uint32_t *>(smem);       // [0, 256) literal bytes | 256 + 64 * table + code
+    uint32_t *bad = h + LZ_HIST_WORDS;
+    for (uint32_t i = tid; i < LZ_HIST_WORDS; i += HIST_NT) h[i] = 0;
+    if (tid == 0) *bad = 0;
+    __syncthreads();
+    const bool cand = W->kind == 0;
+    if (cand) {
+        const uint8_t *lit = wk_lit(P, chunk);
+        for (uint32_t i = tid; i < W->nlit; i += HIST_NT) atomicAdd(&h[lit[i]], 1u);
+        for (int t = 0; t < 3; t++) {
+            const uint8_t *codes = wk_codes(P, chunk, t);
+            for (uint32_t i = tid; i < W->nseq; i += HIST_NT) atomicAdd(&h[256 + 64 * t + (codes[i] & 63u)], 1u);
         }
-        if (W->kind == 0)
-            for (uint32_t i = tid; i < nlit; i += HIST_NT) P.dbg_lits[(uint64_t)chunk * P.blockmax + i] = lit[i];
-    }
-    if (W->kind != 0) return;
-    uint32_t acc0 = 0, acc1 = 0;                       // symbols tid and tid + 128
-    uint8_t *hcol = smem + w * 256 * 32 + lane;
-    for (uint32_t s0 = 0; s0 < nlit; s0 += HIST_SLICE) {
-        const uint32_t s1 = (s0 + HIST_SLICE < nlit) ? s0 + HIST_SLICE : nlit;
-        for (uint32_t i = tid; i < HIST_SMEM_BYTES / 4; i += HIST_NT) reinterpret_cast<uint32_t *>(smem)[i] = 0;
-        __syncthreads();
-        hist_count_stream<255>(lit, s0, s1, hcol, tid);
-        __syncthreads();
-#pragma unroll
-        for (int half = 0; half < 2; half++) {
-            const uint32_t sym = tid + 128 * half;
-            uint32_t c = 0;
-#pragma unroll
-            for (int k = 0; k < HIST_WARPS; k++) {
-                const uint32_t *row = reinterpret_cast<const uint32_t *>(smem + k * 256 * 32 + sym * 32);
-#pragma unroll
-                for (int j = 0; j < 8; j++) {
-                    const uint32_t v = row[(j + (tid >> 2)) & 7];     // rotated: the 32 threads of a warp spread over the banks
-                    c += (v & 0xff) + ((v >> 8) & 0xff) + ((v >> 16) & 0xff) + (v >> 24);
-                }
-            }
-            if (half == 0) acc0 += c; else acc1 += c;
-        }
-        __syncthreads();
-    }
-    W->litHist[tid] = acc0;
-    W->litHist[tid + 128] = acc1;
-    // sequence-code counts: the same private byte counters, one 64-row table per code stream and warp
-    uint32_t cacc = 0, acc1c = 0;                       // code bins tid and tid + 128 (bin = table * 64 + code)
-    const uint8_t *codes = wk_codes(P, chunk, 0);
-    const uint32_t mseq = P.maxseq;
-    for (uint32_t s0 = 0; s0 < nseq; s0 += HIST_SLICE) {
-        const uint32_t s1 = (s0 + HIST_SLICE < nseq) ? s0 + HIST_SLICE : nseq;
-        for (uint32_t i = tid; i < HIST_SMEM_BYTES / 4; i += HIST_NT) reinterpret_cast<uint32_t *>(smem)[i] = 0;
-        __syncthreads();
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-            uint8_t *ccol = smem + w * 256 * 32 + c * 64 * 32 + lane;
-            hist_count_stream<63>(codes + (uint32_t)c * mseq, s0, s1, ccol, tid);      // maxseq is a multiple of 16
-        }
-        __syncthreads();
-        for (uint32_t i = tid; i < 192; i += HIST_NT) {     // (HIST_NT = 128: two rounds; the accumulator is per (round, thread))
-            uint32_t c = 0;
-#pragma unroll
-            for (int k = 0; k < HIST_WARPS; k++) {
-                const uint32_t *row = reinterpret_cast<const uint32_t *>(smem + k * 256 * 32 + i * 32);
-#pragma unroll
-                for (int jj = 0; jj < 8; jj++) {
-                    const uint32_t v = row[(jj + (tid >> 2)) & 7];
-                    c += (v & 0xff) + ((v >> 8) & 0xff) + ((v >> 16) & 0xff) + (v >> 24);
-                }
-            }
-            if (i < HIST_NT) cacc += c; else acc1c += c;
-        }
-        __syncthreads();
-    }
-    uint32_t *shist = reinterpret_cast<uint32_t *>(smem);      // 6 ballot words
-    for (uint32_t i = tid; i < 192; i += HIST_NT) {
-        const uint32_t c = (i < HIST_NT) ? cacc : acc1c;
-        W->seqHist[i / 64][i % 64] = c;
-        // highest used code of each table: index groups of 32 are warp-aligned
-        const unsigned nz = __ballot_sync(FULLMASK, c != 0);
-        if ((i & 31) == 0) shist[i >> 5] = nz;
     }
     __syncthreads();
-    if (tid < 3) {
-        const uint32_t lo = shist[2 * tid], hi = shist[2 * tid + 1];
-        W->maxSym[tid] = hi ? 32 + (31 - (uint32_t)__clz((int)hi)) : (lo ? 31 - (uint32_t)__clz((int)lo) : 0u);
+    if (cand) {
+        for (uint32_t i = tid; i < 256; i += HIST_NT)
+            if (h[i] != W->litHist[i]) *bad = 1;
+        for (uint32_t i = tid; i < 192; i += HIST_NT)
+            if (h[256 + i] != W->seqHist[i / 64][i % 64]) *bad = 1;
+        if (tid < 3) {
+            uint32_t mx = 0;
+            for (uint32_t c = 0; c < 64; c++)
+                if (h[256 + 64 * tid + c]) mx = c;
+            if (mx != W->maxSym[tid]) *bad = 1;
+        }
     }
+    __syncthreads();
+    if (tid == 0 && *bad) W->kind = 3;
     __syncthreads();
 }
+#endif
 
 #ifndef B2C_EMU
 // The parse kernels are persistent (one CTA per resident slot); chunks are handed out through a global counter, so a CTA
@@ -1029,10 +968,6 @@ B2C_LZ_KERNEL(b2c_lz_snappy_fast_kernel, 3, LZ_MODE_SNAPPY)
 B2C_LZ_KERNEL(b2c_lz_s2_better_kernel, 4, LZ_MODE_S2)
 B2C_LZ_KERNEL(b2c_lz_snappy_better_kernel, 4, LZ_MODE_SNAPPY)
 #undef B2C_LZ_KERNEL
-extern "C" __global__ void __launch_bounds__(HIST_NT) b2c_zstd_hist_kernel(ZstdEncParams P) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    for (uint32_t c = blockIdx.x; c < P.nchunks; c += gridDim.x) zstd_hist_chunk(smem, P, c);
-}
 #endif
 
 }  // namespace b2c

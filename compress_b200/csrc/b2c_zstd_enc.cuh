@@ -7,10 +7,10 @@
 //   zstd/frameenc.go:25-92    frameHeader.appendTo
 //   zstd/internal/xxhash      XXH64 frame checksum
 //
-// B200-first design: a pipeline of six kernels on one stream, each shaped after the parallelism its stage really has, with
+// B200-first design: a pipeline of four kernels on one stream, each shaped after the parallelism its stage really has, with
 // a per-chunk work record (ChunkWork header + a slab of the work pool) in HBM/L2 between them:
-//   K1 parse    b2c_lz.cuh: the tile-ordered match finder (levels 1-3; also the S2 / Snappy block encoders)
-//   hist        b2c_lz.cuh: literal and sequence-code histograms
+//   K1 parse    b2c_lz.cuh: the tile-ordered match finder (levels 1-3; also the S2 / Snappy block encoders), with the
+//               literal and sequence-code histograms counted as the literals and codes are written
 //   K2 tables   one 4-warp CTA per chunk: the Huffman table (reference tie-breaking) and the three FSE
 //               tables are tiny serial problems -- thousands of them run side by side.
 //   K3 chains   one LANE per (chunk, tANS chain): the reference's serial state walk, 32 chunks per warp.
@@ -288,8 +288,22 @@ struct TablesShared {
 B2C_DEV void zstd_tables_chunk(TablesShared *ts, const ZstdEncParams &P, uint32_t chunk) {
     const unsigned tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
     ChunkWork *W = P.work + chunk;
-    if (W->kind != 0) return;
     const uint32_t nseq = W->nseq, nlit = W->nlit;
+    if (P.dbg_hdr && W->kind != 3) {
+        // debug dump of the parse (tests): the sequences (of raw blocks too) and the literals of compressed candidates
+        const WkLens wlen = wk_lens(P, chunk);
+        const uint32_t *wof = wk_of(P, chunk);
+        for (uint32_t i = tid; i < nseq && i < P.dbg_seq_cap && i < P.maxseq; i += TABLES_NT) {
+            uint32_t *d = P.dbg_seqs + ((uint64_t)chunk * P.dbg_seq_cap + i) * 3;
+            d[0] = wlen.get_ll(i); d[1] = wlen.get_ml(i); d[2] = wof[i];
+        }
+        if (W->kind == 0) {
+            const uint8_t *lit = wk_lit(P, chunk);
+            for (uint32_t i = tid; i < nlit; i += TABLES_NT) P.dbg_lits[(uint64_t)chunk * P.blockmax + i] = lit[i];
+        }
+    }
+    if (P.dbg_hdr) __syncthreads();      // every warp has read the parse's kind before a table error may change it
+    if (W->kind != 0) return;
     if (w == 0) {
         HufWork *hw = &ts->hw;
         for (uint32_t s = lane; s < 256; s += 32) hw->count[s] = W->litHist[s];

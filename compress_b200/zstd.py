@@ -68,6 +68,8 @@ class Encoder:
     def sm_count(self):
         return int(lib.b2c_sm_count(self._ctx))
 
+    # profile slots of b2c_profile_read.  The histograms are counted inside the parse kernel, so the
+    # "b2c_zstd_hist_kernel" slot is an empty interval (about 0 ms); the key stays so that readers of the profile keep working.
     KERNELS = ("b2c_zstd_xxh_kernel", "b2c_lz_parse_kernel", "b2c_zstd_hist_kernel", "b2c_zstd_tables_kernel",
                "b2c_zstd_chains_kernel", "b2c_zstd_pack_kernel")
 

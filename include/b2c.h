@@ -81,7 +81,8 @@ B2C_API uint64_t b2c_launch_count(b2c_ctx *ctx);
 /* Per-kernel timing of the encode pipeline with CUDA events recorded on the launching stream (bench.py's
  * roofline).  b2c_profile_enable(ctx, 1) starts collecting; b2c_profile_read synchronises the device and returns in
  * ms[0..5] the summed durations of {xxh64, parse, histograms, tables, chains, pack} over the *ncalls encode launches
- * since (a device-resident call larger than the work pool is several launches). */
+ * since (a device-resident call larger than the work pool is several launches).  The histograms are counted inside the
+ * parse kernel, so ms[2] is an empty interval (about 0 ms), kept so that the slots keep their meaning. */
 B2C_API int b2c_profile_enable(b2c_ctx *ctx, int on);
 B2C_API int b2c_profile_read(b2c_ctx *ctx, double *ms, uint32_t *ncalls);
 /* The same for zstd decode: ms[0..5] = {scan, literals, sequences, execute, xxh64, one-warp decoder} summed over the decode
